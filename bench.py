@@ -323,7 +323,12 @@ def main():
                          "E = configs[4] per GPU (128 sequences, 400 tracks, 50-pose window, 20 SLAM features)")
     ap.add_argument("--streams", type=int, default=4,
                     help="sub-batches per GPU, each an independent handle/stream driven by its own host thread")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the run, write what the last timed step of each timed pass returned (publish flags, filter states of "
+                         "every sequence) as DIR/<name>.npy in float64, so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.warmup < 3:
@@ -419,6 +424,8 @@ def main():
         return bs
 
     batches = make_batches()
+    last_pub = [None] * NSUB              # what the newest step of sub-batch i returned to its caller
+    last_states = [None] * NSUB
     frames_host = np.stack([np.stack([seqs[s].images[j] for s in range(S)]) for j in range(n_frames)])   # [F][S][H][W]
     pinned = torch.from_numpy(frames_host).pin_memory()
     t_img = np.stack([[seqs[s].img_t[j] for s in range(S)] for j in range(n_frames)])
@@ -455,10 +462,10 @@ def main():
             imu["t"][rr, cc] = arr[:, :, 0][valid]; imu["gyro"][rr, cc] = arr[:, :, 1:4][valid]; imu["acc"][rr, cc] = arr[:, :, 4:7][valid]
             n_imu += m.astype(np.int32)
             if mode == "dev":
-                bb.step(dev_frames[j, lo:hi].data_ptr(), t_img[j, lo:hi], imu, n_imu, images_on_device=True)
+                last_pub[i] = bb.step(dev_frames[j, lo:hi].data_ptr(), t_img[j, lo:hi], imu, n_imu, images_on_device=True)
             else:
-                bb.step(pinned[j, lo:hi].numpy(), t_img[j, lo:hi], imu, n_imu)
-                bb.get_states()
+                last_pub[i] = bb.step(pinned[j, lo:hi].numpy(), t_img[j, lo:hi], imu, n_imu)
+                last_states[i] = bb.get_states()
 
     def run_pass(mode, lo_f, hi_f, state):
         if NSUB == 1:
@@ -506,6 +513,9 @@ def main():
     e1.record(); torch.cuda.synchronize(); wall = time.perf_counter() - t0
     ms_dev = max(e0.elapsed_time(e1), 1e3 * wall * 0.0)     # each step ends with a stream sync, so events == wall
     barrier()
+    dump = {}
+    if args.dump_outputs:
+        dump.update(published=np.concatenate(last_pub), states=all_states())
     clocks = sampler.stop() if sampler else None
     launches = launches_total() - l0
     # steady-state evidence: sliding-window fill and state dimension of every sequence right after the timed region
@@ -539,6 +549,8 @@ def main():
     run_pass("e2e", PR + Wm, PR + Wm + K, st)
     e3.record(); torch.cuda.synchronize(); wall_e2e = time.perf_counter() - t0
     ms_e2e = max(e2.elapsed_time(e3), 0.0)
+    if args.dump_outputs:
+        dump.update(e2e_published=np.concatenate(last_pub), e2e_states=np.concatenate(last_states))
     t = torch.tensor([ms_dev, ms_e2e], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -619,6 +631,10 @@ def main():
                     gpu_launches=int(launches), clocks=clocks, roofline=roof, kernels=kernel_share, kernel_rooflines=roofs, work_counters=pstats,
                     steady_state=steady, lk_paths=lk_paths, ekf_update_ms=ekf_ms, step_roofline=step_roof, cpu_baseline=cpu_baseline, gen_seconds=t_gen, wall_dev_s=wall, wall_e2e_s=wall_e2e)
         print(json.dumps(line))
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(arr, np.float64))
     if world > 1:
         dist.destroy_process_group()
     return 0

@@ -799,10 +799,7 @@ def test_unsupported_configs_fail_loudly(lib_built):
 
 # ---- the CUDA back end against golden vectors the REFERENCE ITSELF produced (tests/golden/ref_*.npz) ---------------------------------
 REF_CASES_GPU = ["msckf_sw30", "msckf_oldest", "hybrid_1d_oldest", "hybrid_3d", "config_d", "zupt", "self_start", "no_fej_no_calib", "calib_3d", "schmidt_1d_oldest",
-                 "schmidt_3d_oldest"]
-# written after the round's GPU minutes were spent (every case above ran green on a B200, profiles/r2q_*, r2r_*): the oracle matches this
-# fixture on CPU, the device has not replayed it yet - a failure here is a finding, not a regression
-REF_CASES_GPU_UNRUN = ["hybrid_zupt", "self_start_jump"]
+                 "schmidt_3d_oldest", "hybrid_zupt", "self_start_jump"]
 
 
 def _drive_fixture(name):
@@ -865,8 +862,7 @@ def _drive_fixture(name):
     return w
 
 
-@pytest.mark.parametrize("name", REF_CASES_GPU + [pytest.param(n, marks=pytest.mark.xfail(strict=False, reason="first GPU run is the driver's"))
-                                                  for n in REF_CASES_GPU_UNRUN])
+@pytest.mark.parametrize("name", REF_CASES_GPU)
 def test_backend_matches_the_compiled_reference(name, lib_built):
     """The CUDA filter against the REFERENCE's own answers (not the numpy oracle): fixtures made by /root/reference/src/larvio.cpp
     compiled unmodified (oracle/_ref, tests/golden/make_ref_golden.py).  Per call: same return value, state dimension and IMU
@@ -934,7 +930,6 @@ def test_shim_facade_matches_the_whole_reference_pipeline(tmp_path, lib_built):
     assert w["n"] >= 60 and w["n_lists"] >= 2 and w["t"] < 1e-9 and max(w["R"], w["p"], w["v"]) < 1e-8 and w["pts"] < 1e-7, w
 
 
-@pytest.mark.xfail(strict=False, reason="written after the round's GPU minutes were spent: first GPU run is the driver's")
 def test_replay_tool_writes_the_file_the_reference_writes(tmp_path, lib_built):
     """SURVEY 8(f-4), both directions of the on-disk formats: larvio_b200/bin/larvio_replay reads the EuRoC ASL directory (PNG + csv)
     and writes msckf_2_state.txt / msckf_2_takeoff.txt; the reference's own LarVio wrote the same two files while its whole
