@@ -189,6 +189,9 @@ long long lvbm_launch_count(const LvbMulti* m);
  * (no padding): clahe [n][H][W], l1 [n][H1][W1], l2 [n][H2][W2], blur [n][H][W]. Any may be NULL. */
 int lvbk_pyramid(LvbHandle* h, const uint8_t* images, int n, uint8_t* clahe, uint8_t* l1, uint8_t* l2,
                  uint8_t* blur);
+/* The same pyramid, one level WITH its REFLECT_101 pad (the LK kernel reads up to 24 px outside a level):
+ * out [n][h + 48][w + 48] for level `level` (0 = the equalised image). */
+int lvbk_pyramid_padded(LvbHandle* h, const uint8_t* images, int n, int level, uint8_t* out);
 /* calcOpticalFlowPyrLK(prev->next, USE_INITIAL_FLOW) on raw (already equalised) image pairs:
  * prev/next [n][H][W]; pts [n][m][2]; status [n][m]. next_pts is in/out (initial flow). */
 int lvbk_lk(LvbHandle* h, const uint8_t* prev, const uint8_t* next, int n, int m, const float* prev_pts,

@@ -67,17 +67,19 @@ _lib.lvb_get_stats.restype = C.c_int
 _lib.lvb_debug_icore.argtypes = [_vp, C.c_int, C.POINTER(C.c_int)]
 _lib.lvb_debug_icore.restype = C.c_int
 _lib.lvb_profile_get.argtypes = [_vp, C.POINTER(C.c_char_p), C.POINTER(C.c_double), C.POINTER(C.c_longlong), C.c_int]
-for _name in ("lvbk_pyramid", "lvbk_lk", "lvbk_orb", "lvbk_detect", "lvbk_undistort", "lvbk_ransac",
+for _name in ("lvbk_pyramid", "lvbk_pyramid_padded", "lvbk_lk", "lvbk_orb", "lvbk_detect", "lvbk_undistort", "lvbk_ransac",
               "lvb_process_images", "lvb_process_features", "lvb_step", "lvb_set_initial_state",
               "lvb_get_state", "lvb_get_states", "lvb_get_window", "lvb_get_covariance", "lvb_get_calibration", "lvb_get_points"):
     if hasattr(_lib, _name):
         getattr(_lib, _name).restype = C.c_int
 
+LVB_PAD = 24          # pyramid level pad (lvb_internal.h)
+
 EXPORTED_SYMBOLS = [
     "lvb_parse_config", "lvb_create", "lvb_create_from_file", "lvb_destroy", "lvb_last_error",
     "lvb_feature_capacity", "lvb_n_seq", "lvb_process_images", "lvb_process_features", "lvb_step",
     "lvb_synchronize", "lvb_set_initial_state", "lvb_get_state", "lvb_get_states", "lvb_get_window",
-    "lvb_get_covariance", "lvb_get_calibration", "lvb_static_init_create", "lvb_static_init_destroy", "lvb_static_init_try", "lvbk_pyramid", "lvbk_lk", "lvbk_orb", "lvbk_detect", "lvbk_undistort",
+    "lvb_get_covariance", "lvb_get_calibration", "lvb_static_init_create", "lvb_static_init_destroy", "lvb_static_init_try", "lvbk_pyramid", "lvbk_pyramid_padded", "lvbk_lk", "lvbk_orb", "lvbk_detect", "lvbk_undistort",
     "lvbk_ransac", "lvb_launch_count", "lvb_profile_enable", "lvb_profile_reset", "lvb_profile_get", "lvb_get_stats", "lvb_debug_icore",
     "lvb_get_points", "lvbm_create", "lvbm_destroy", "lvbm_n_shards", "lvbm_set_initial_state", "lvbm_step", "lvbm_get_states",
     "lvbm_launch_count",
@@ -239,6 +241,16 @@ class Batch:
         blur = np.empty((n, H, W), np.uint8)
         _check(_lib.lvbk_pyramid(self._h, _p(images), n, _p(clahe), _p(l1), _p(l2), _p(blur)))
         return clahe, l1, l2, blur
+
+    def k_pyramid_padded(self, images: np.ndarray, level: int):
+        """Level `level` of the pyramid with its REFLECT_101 pad of LVB_PAD pixels: [n][h + 2 LVB_PAD][w + 2 LVB_PAD]."""
+        images = np.ascontiguousarray(images, np.uint8)
+        n, h, w = images.shape
+        for _ in range(level):
+            h, w = (h + 1) // 2, (w + 1) // 2
+        out = np.empty((n, h + 2 * LVB_PAD, w + 2 * LVB_PAD), np.uint8)
+        _check(_lib.lvbk_pyramid_padded(self._h, _p(images), n, int(level), _p(out)))
+        return out
 
     def k_lk(self, prev: np.ndarray, nxt: np.ndarray, prev_pts: np.ndarray, init_pts: np.ndarray):
         prev = np.ascontiguousarray(prev, np.uint8); nxt = np.ascontiguousarray(nxt, np.uint8)

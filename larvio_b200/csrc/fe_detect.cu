@@ -13,15 +13,12 @@
 
 namespace {
 
-constexpr int TW = 32, TH = 16;           // output tile
-constexpr int CW = TW + 2, CH = TH + 2;   // cov grid (box apron 1)
-constexpr int IW = TW + 4, IH = TH + 4;   // image tile (Sobel apron 1 more)
-
-__device__ __forceinline__ int reflect101(int p, int n) {
-  if (p < 0) p = -p;
-  if (p >= n) p = 2 * n - 2 - p;
-  return p;
-}
+constexpr int TW = 64, TH = 16;           // output tile
+constexpr int RW = TW + 2, RH = TH + 2;   // response grid (non-maximum apron 1)
+constexpr int PW = TW + 4, PH = TH + 4;   // product grid (box apron 1 more)
+constexpr int LW = TW + 8, LH = TH + 6;   // image tile (Sobel apron 1 more), whole 32-bit words from bx - 4
+constexpr int STRIP = 6;                  // response rows per thread in the column-sum stage (RH / STRIP strips per column)
+static_assert(RH % STRIP == 0 && RW * (RH / STRIP) <= 256, "one column strip per thread");
 
 __device__ __forceinline__ int float_order_key(float v) {
   int b = __float_as_int(v);
@@ -34,21 +31,24 @@ struct CornerArgs {
   float* eig;              // [S][H][W] or null: the response map is only written for the stage-level test entry point
   int* eig_max_key;        // [S] ordered-int key of the masked maximum
   unsigned long long* cand; int* n_cand; int cap;
+  int* hist;               // [S][LVB_CAND_BINS] candidates per value-bits bin
   const int* enable;       // [S] or null
 };
 
 // cornerMinEigenVal + the masked maximum + the 3x3 non-maximum test in ONE pass over the level (SURVEY F5: the image is read
 // once; the f32 response map of the two-kernel version - 1.4 MB per sequence written and re-read - no longer exists).
-// A tile computes the response on its 32x16 outputs plus a one-pixel apron (neighbours of the non-maximum test), from the
-// covariance products on a 36x20 grid and the image on 38x22.  The 3x3 box is separable: row sums, then column sums, in
-// double like OpenCV's RowSum<float,double> / ColumnSum<double,float>, 12 DADD per pixel instead of 24.
+// A tile computes the response on its 64x16 outputs plus a one-pixel apron (neighbours of the non-maximum test), from the
+// covariance products on a 68x20 grid and the image on 70x22 (staged as 72x22 in aligned words).  The products are widened
+// to double once, where they are made; the 3x3 box is separable - row sums, then column sums, in double like OpenCV's
+// RowSum<float,double> / ColumnSum<double,float> - and a thread walks a 6-row strip of one response column, so each row sum
+// of the strip is made once, in registers.
 // The global threshold 0.01 * max is not known yet, so a tile keeps every local maximum above 0.01 * (its own masked
-// maximum) - a lower bound of the final threshold - and select_kernel applies the exact one.
+// maximum) - a lower bound of the final threshold - and select_kernel applies the exact one.  Every candidate is also counted
+// in its sequence's value histogram (LVB_CAND_BINS bins of the float bits), from which select_kernel cuts its chunks.
 __global__ void __launch_bounds__(256) corner_kernel(CornerArgs a) {
-  __shared__ uint8_t img[IH + 2][IW + 6];                 // 22 x 44 (38 used)
-  __shared__ float sxx[CH + 2][CW + 2], sxy[CH + 2][CW + 2], syy[CH + 2][CW + 2];      // products on the 36 x 20 grid
-  __shared__ double hxx[CH + 2][CW], hxy[CH + 2][CW], hyy[CH + 2][CW];                // row sums on 34 x 20
-  __shared__ float se[CH][CW];                            // response on 34 x 18
+  __shared__ uint32_t imgw[LH][LW / 4];                   // image tile: byte (tx, ty) <-> pixel (bx - 4 + tx, by - 3 + ty)
+  __shared__ double pxx[PH][PW], pxy[PH][PW], pyy[PH][PW];  // products: cell (cx, cy) <-> pixel (bx - 2 + cx, by - 2 + cy)
+  __shared__ float se[RH][RW];                            // response: cell (ex, ey) <-> pixel (bx - 1 + ex, by - 1 + ey)
   __shared__ int blk_max;
   const int s = blockIdx.z;
   if (a.enable && !a.enable[s]) return;
@@ -57,34 +57,35 @@ __global__ void __launch_bounds__(256) corner_kernel(CornerArgs a) {
   const int bx = blockIdx.x * TW, by = blockIdx.y * TH;
   const uint8_t* org = lvb_level_origin(a.pyr, a.L, s, 0);
   const int tid = threadIdx.x;
-  constexpr int PW = CW + 2, PH = CH + 2;                 // product grid 36 x 20: cell (cx, cy) <-> pixel (bx - 2 + cx, by - 2 + cy)
-  constexpr int LW = IW + 2, LH = IH + 2;                 // image tile 38 x 22: (tx, ty) <-> pixel (bx - 3 + tx, by - 3 + ty)
   if (tid == 0) blk_max = INT_MIN;
-  for (int i = tid; i < LH * LW; i += 256) {
-    const int ty = i / LW, tx = i - ty * LW;
-    int gx = bx - 3 + tx, gy = by - 3 + ty;
-    gx = min(gx, W + LVB_PAD - 1); gy = min(gy, H + LVB_PAD - 1);
-    img[ty][tx] = org[(ptrdiff_t)gy * lv.pitch + gx];
+  // the level origin is 8-byte aligned and bx - 4 a multiple of 4; clamped words (only read for cells that are never used)
+  // stay inside the padded rows
+  for (int i = tid; i < LH * (LW / 4); i += 256) {
+    const int ty = i / (LW / 4), wq = i - ty * (LW / 4);
+    const int gy = min(by - 3 + ty, H + LVB_PAD - 1);
+    const int gx = min(bx - 4 + 4 * wq, lv.pitch - LVB_PAD - 4);
+    imgw[ty][wq] = *reinterpret_cast<const uint32_t*>(org + (ptrdiff_t)gy * lv.pitch + gx);
   }
   __syncthreads();
+  const uint8_t* img = reinterpret_cast<const uint8_t*>(&imgw[0][0]);
   const double scale = 1.0 / (4.0 * 3.0 * 255.0);
   const float k0 = (float)(2.0 * scale), k1 = (float)scale;
   const int tail_x = W & ~31;
   for (int i = tid; i < PH * PW; i += 256) {
     const int cy = i / PW, cx = i - cy * PW;
-    if (bx - 2 + cx > W || by - 2 + cy > H) { sxx[cy][cx] = 0.f; sxy[cy][cx] = 0.f; syy[cy][cx] = 0.f; continue; }
-    const int gx = reflect101(bx - 2 + cx, W), gy = reflect101(by - 2 + cy, H);   // the box filter's REFLECT_101 is on the products
-    const int tx = gx - (bx - 3), ty = gy - (by - 3);     // position inside img[][]
+    if (bx - 2 + cx > W || by - 2 + cy > H) { pxx[cy][cx] = 0.0; pxy[cy][cx] = 0.0; pyy[cy][cx] = 0.0; continue; }
+    const int gx = lvb_reflect101(bx - 2 + cx, W), gy = lvb_reflect101(by - 2 + cy, H);   // the box filter's REFLECT_101 is on the products
+    const uint8_t* m = img + (gy - (by - 3)) * LW + (gx - (bx - 4));              // the pixel inside the tile
     // Dx: row diff then symmetric column filter with FMA
-    const float d0 = (float)((int)img[ty - 1][tx + 1] - (int)img[ty - 1][tx - 1]);
-    const float d1 = (float)((int)img[ty][tx + 1] - (int)img[ty][tx - 1]);
-    const float d2 = (float)((int)img[ty + 1][tx + 1] - (int)img[ty + 1][tx - 1]);
+    const float d0 = (float)((int)m[-LW + 1] - (int)m[-LW - 1]);
+    const float d1 = (float)((int)m[1] - (int)m[-1]);
+    const float d2 = (float)((int)m[LW + 1] - (int)m[LW - 1]);
     const float Dx = __fmaf_rn(__fadd_rn(d0, d2), k1, __fmul_rn(d1, k0));
     // Dy: smoothing row filter (FMA chain; plain mul/add in the last W%32 columns), then row diff
     float r0, r2;
     {
-      const float a0 = (float)img[ty - 1][tx - 1], a1 = (float)img[ty - 1][tx], a2 = (float)img[ty - 1][tx + 1];
-      const float b0 = (float)img[ty + 1][tx - 1], b1 = (float)img[ty + 1][tx], b2 = (float)img[ty + 1][tx + 1];
+      const float a0 = (float)m[-LW - 1], a1 = (float)m[-LW], a2 = (float)m[-LW + 1];
+      const float b0 = (float)m[LW - 1], b1 = (float)m[LW], b2 = (float)m[LW + 1];
       if (gx < tail_x) {
         r0 = __fmaf_rn(a2, k1, __fmaf_rn(a1, k0, __fmul_rn(a0, k1)));
         r2 = __fmaf_rn(b2, k1, __fmaf_rn(b1, k0, __fmul_rn(b0, k1)));
@@ -94,34 +95,37 @@ __global__ void __launch_bounds__(256) corner_kernel(CornerArgs a) {
       }
     }
     const float Dy = __fsub_rn(r2, r0);
-    sxx[cy][cx] = __fmul_rn(Dx, Dx);
-    sxy[cy][cx] = __fmul_rn(Dx, Dy);
-    syy[cy][cx] = __fmul_rn(Dy, Dy);
+    pxx[cy][cx] = (double)__fmul_rn(Dx, Dx);
+    pxy[cy][cx] = (double)__fmul_rn(Dx, Dy);
+    pyy[cy][cx] = (double)__fmul_rn(Dy, Dy);
   }
   __syncthreads();
-  // row sums: h[cy][ex] = p[cy][ex] + p[cy][ex + 1] + p[cy][ex + 2]   (ex over the 34 response columns)
-  for (int i = tid; i < PH * CW; i += 256) {
-    const int cy = i / CW, ex = i - cy * CW;
-    hxx[cy][ex] = ((double)sxx[cy][ex] + (double)sxx[cy][ex + 1]) + (double)sxx[cy][ex + 2];
-    hxy[cy][ex] = ((double)sxy[cy][ex] + (double)sxy[cy][ex + 1]) + (double)sxy[cy][ex + 2];
-    hyy[cy][ex] = ((double)syy[cy][ex] + (double)syy[cy][ex + 1]) + (double)syy[cy][ex + 2];
-  }
-  __syncthreads();
-  // column sums + min eigenvalue on the 34 x 18 response grid: cell (ex, ey) <-> pixel (bx - 1 + ex, by - 1 + ey)
-  for (int i = tid; i < CH * CW; i += 256) {
-    const int ey = i / CW, ex = i - ey * CW;
-    const double xx = (hxx[ey][ex] + hxx[ey + 1][ex]) + hxx[ey + 2][ex];
-    const double xy = (hxy[ey][ex] + hxy[ey + 1][ex]) + hxy[ey + 2][ex];
-    const double yy = (hyy[ey][ex] + hyy[ey + 1][ex]) + hyy[ey + 2][ex];
-    const float fa = __fmul_rn((float)xx, 0.5f), fb = (float)xy, fc = __fmul_rn((float)yy, 0.5f);
-    const float dif = __fsub_rn(fa, fc);
-    se[ey][ex] = __fsub_rn(__fadd_rn(fa, fc), __fsqrt_rn(__fadd_rn(__fmul_rn(dif, dif), __fmul_rn(fb, fb))));
+  // row sums h[cy][ex] = (p[cy][ex] + p[cy][ex + 1]) + p[cy][ex + 2], column sums (h[ey] + h[ey + 1]) + h[ey + 2], min eigenvalue
+  if (tid < RW * (RH / STRIP)) {
+    const int ex = tid % RW, ey0 = (tid / RW) * STRIP;
+    double hx[3], hy[3], hz[3];
+#pragma unroll
+    for (int r = 0; r < STRIP + 2; ++r) {
+      const int cy = ey0 + r;
+      hx[r % 3] = (pxx[cy][ex] + pxx[cy][ex + 1]) + pxx[cy][ex + 2];
+      hy[r % 3] = (pxy[cy][ex] + pxy[cy][ex + 1]) + pxy[cy][ex + 2];
+      hz[r % 3] = (pyy[cy][ex] + pyy[cy][ex + 1]) + pyy[cy][ex + 2];
+      if (r >= 2) {
+        const double xx = (hx[(r - 2) % 3] + hx[(r - 1) % 3]) + hx[r % 3];
+        const double xy = (hy[(r - 2) % 3] + hy[(r - 1) % 3]) + hy[r % 3];
+        const double yy = (hz[(r - 2) % 3] + hz[(r - 1) % 3]) + hz[r % 3];
+        const float fa = __fmul_rn((float)xx, 0.5f), fb = (float)xy, fc = __fmul_rn((float)yy, 0.5f);
+        const float dif = __fsub_rn(fa, fc);
+        se[ey0 + r - 2][ex] = __fsub_rn(__fadd_rn(fa, fc), __fsqrt_rn(__fadd_rn(__fmul_rn(dif, dif), __fmul_rn(fb, fb))));
+      }
+    }
   }
   __syncthreads();
   // masked maximum of this tile
-  float myv[2]; bool mym[2]; int my_key = INT_MIN;
+  constexpr int PER = TW * TH / 256;
+  float myv[PER]; bool mym[PER]; int my_key = INT_MIN;
 #pragma unroll
-  for (int r = 0; r < 2; ++r) {
+  for (int r = 0; r < PER; ++r) {
     const int i = tid + 256 * r;
     const int oy = i / TW, ox = i - oy * TW;
     const int gx = bx + ox, gy = by + oy;
@@ -145,7 +149,7 @@ __global__ void __launch_bounds__(256) corner_kernel(CornerArgs a) {
   const float tile_max = __int_as_float(key >= 0 ? key : (key ^ 0x7fffffff));
   const float thr_lo = (float)((double)tile_max * 0.01);  // <= the final threshold (float)(0.01 * global max): same monotone rounding
 #pragma unroll
-  for (int r = 0; r < 2; ++r) {
+  for (int r = 0; r < PER; ++r) {
     const int i = tid + 256 * r;
     const int oy = i / TW, ox = i - oy * TW;
     const int gx = bx + ox, gy = by + oy;
@@ -165,17 +169,26 @@ __global__ void __launch_bounds__(256) corner_kernel(CornerArgs a) {
       base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
       if (is) {
         const int pos = base + __popc(m & ((1u << lane) - 1));
-        if (pos < a.cap)
-          a.cand[(size_t)s * a.cap + pos] = ((unsigned long long)(unsigned)__float_as_int(v) << 32) | (unsigned)(gy * W + gx);
+        const unsigned bits = (unsigned)__float_as_int(v);
+        if (pos < a.cap) a.cand[(size_t)s * a.cap + pos] = ((unsigned long long)bits << 32) | (unsigned)(gy * W + gx);
+        atomicAdd(&a.hist[(size_t)s * LVB_CAND_BINS + (bits >> 19)], 1);
       }
     }
   }
 }
 
 // ---------------------------------------------------------------- per-sequence select: top-K chunks, sort, greedy
+// Candidates are taken in chunks of consecutive descending keys; the greedy pass continues across chunks, so where a chunk
+// ends does not change the result.  A chunk is cut at a histogram bin boundary: the bins below the previous cut are scanned
+// from the top until they hold about CHUNK_TARGET candidates (never more than CHUNK).  Only a single bin that alone holds
+// more than CHUNK is refined, by bisection over the value bits of that bin.
 constexpr int CHUNK = 4096;
+constexpr int CHUNK_TARGET = 1024;
+constexpr int BIN_SHIFT = 19;                 // value bits >> BIN_SHIFT: LVB_CAND_BINS bins over the positive floats
+static_assert((0x7fffffffu >> BIN_SHIFT) + 1 == LVB_CAND_BINS, "bins cover bits 30..BIN_SHIFT");
 struct SelArgs {
   const unsigned long long* cand; const int* n_cand; int cap;
+  const int* hist;          // [S][LVB_CAND_BINS]
   const int* want; int W; int min_dist; int stride;
   float2* out; int* out_n; int* overflow;
   const int* enable;
@@ -184,8 +197,8 @@ struct SelArgs {
 
 __global__ void __launch_bounds__(1024) select_kernel(SelArgs a) {
   __shared__ unsigned long long keys[CHUNK];
-  __shared__ int s_cnt, s_acc, s_done;
-  __shared__ unsigned long long s_upper;
+  __shared__ int s_cnt, s_acc, s_done, s_rover, s_rtgt, s_pover;
+  __shared__ unsigned s_upper;                  // value bits: the keys still to be taken are those below s_upper << 32
   __shared__ short2 accepted[512];
   __shared__ int red[32];
   const int s = blockIdx.x;
@@ -195,64 +208,104 @@ __global__ void __launch_bounds__(1024) select_kernel(SelArgs a) {
   const int want = min(a.want[s], min(a.stride, 512));
   if (n > a.cap) { if (tid == 0) atomicExch(a.overflow, 1); n = a.cap; }
   const unsigned long long* c = a.cand + (size_t)s * a.cap;
-  if (tid == 0) { s_acc = 0; s_done = 0; s_upper = ~0ull; }
+  const int* hist = a.hist + (size_t)s * LVB_CAND_BINS;
+  if (tid == 0) { s_acc = 0; s_done = 0; s_upper = 0x80000000u; s_rover = INT_MAX; s_rtgt = INT_MAX; }
   __syncthreads();
   if (want <= 0 || n <= 0) { if (tid == 0) a.out_n[s] = 0; return; }
   const int md2 = a.min_dist * a.min_dist;
-  // v > thr for positive floats <=> value bits > thr bits <=> key >= (thr bits + 1) << 32
-  unsigned long long lowk = 0ull;
+  // v > thr for positive floats <=> value bits > thr bits <=> value bits >= lowb
+  unsigned lowb = 0u;
   {
     const int key = a.eig_max_key[s];
     if (key == INT_MIN) { if (tid == 0) a.out_n[s] = 0; return; }
     const float maxv = __int_as_float(key >= 0 ? key : (key ^ 0x7fffffff));
     const float thr = (float)((double)maxv * 0.01);
     if (!(thr >= 0.f)) { if (tid == 0) a.out_n[s] = 0; return; }       // no positive response anywhere: no corner
-    lowk = ((unsigned long long)(unsigned)__float_as_int(thr) + 1ull) << 32;
+    lowb = (unsigned)__float_as_int(thr) + 1u;
   }
-  while (true) {
-    const unsigned long long upper = s_upper;
-    // --- bisection on the value bits: smallest cut with count{cut<<32 <= k < upper} <= CHUNK
-    unsigned long long lo = 0ull, hi = (upper >> 32) + 1ull;   // count(k >= hi<<32, k < upper) == 0
-    for (int it = 0; it < 40; ++it) {
-      const unsigned long long mid = (it == 0) ? 0ull : lo + ((hi - lo) >> 1);
-      const unsigned long long midk = max(mid << 32, lowk);
-      int cnt = 0;
-      for (int i = tid; i < n; i += 1024) { const unsigned long long k = c[i]; cnt += (k >= midk && k < upper); }
+  // exact count of the keys with value bits in [lo, upper), block-wide
+  auto count_from = [&](unsigned lo, unsigned upper) -> int {
+    const unsigned long long lok = (unsigned long long)lo << 32, upk = (unsigned long long)upper << 32;
+    int cnt = 0;
+    for (int i = tid; i < n; i += 1024) { const unsigned long long k = c[i]; cnt += (k >= lok && k < upk); }
 #pragma unroll
-      for (int o = 16; o; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-      if ((tid & 31) == 0) red[tid >> 5] = cnt;
-      __syncthreads();
-      if (tid < 32) {
-        int v = red[tid];
+    for (int o = 16; o; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if ((tid & 31) == 0) red[tid >> 5] = cnt;
+    __syncthreads();
+    if (tid < 32) {
+      int v = red[tid];
 #pragma unroll
-        for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (tid == 0) s_cnt = v;
-      }
-      __syncthreads();
-      const int total = s_cnt;
-      __syncthreads();
-      if (it == 0) {
-        if (total <= CHUNK) { hi = 0ull; break; }
-        continue;
-      }
-      if (total <= CHUNK) hi = mid; else lo = mid;
-      if (hi - lo <= 1) break;
+      for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if (tid == 0) s_cnt = v;
     }
-    const unsigned long long cut = max(hi << 32, lowk);
+    __syncthreads();
+    const int total = s_cnt;
+    __syncthreads();
+    return total;
+  };
+  const int bL = (int)(lowb >> BIN_SHIFT);
+  while (true) {
+    const unsigned upper = s_upper;
+    // --- histogram scan: bins bU (holding upper - 1) down to bL, ranked from the top; thread t owns ranks 4t .. 4t+3.
+    // A bin's count includes keys outside [lowb, upper) only in the two end bins, so every prefix is an upper bound.
+    const int bU = (int)((upper - 1u) >> BIN_SHIFT), nr = bU - bL + 1;
+    int hv[4], run = 0;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) { const int r = 4 * tid + q; hv[q] = r < nr ? hist[bU - r] : 0; run += hv[q]; }
+    int x = run;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if ((tid & 31) >= o) x += y; }
+    if ((tid & 31) == 31) red[tid >> 5] = x;
+    __syncthreads();
+    int pre = x - run;
+    for (int w = 0; w < (tid >> 5); ++w) pre += red[w];
+    // the first rank whose prefix exceeds CHUNK (and the prefix above it), the first rank whose prefix reaches CHUNK_TARGET
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int r = 4 * tid + q, above = pre;
+      pre += hv[q];
+      if (r < nr && pre > CHUNK && above <= CHUNK) { s_rover = r; s_pover = above; }
+      if (r < nr && pre >= CHUNK_TARGET && above < CHUNK_TARGET) s_rtgt = r;
+    }
+    __syncthreads();
+    const int r_over = min(s_rover, nr), r_tgt = min(s_rtgt, nr - 1), p_over = s_pover;
+    const int r_cut = min(r_over - 1, r_tgt);     // the chunk is ranks 0 .. r_cut
+    unsigned cut;
+    if (r_over < nr && r_cut == r_over - 1 && p_over == 0) {
+      // rank r_over alone holds more than CHUNK, nothing above it: bisect inside that bin for the smallest cut that fits
+      const unsigned b = (unsigned)(bU - r_over);
+      unsigned lo = max(b << BIN_SHIFT, lowb), hi = min(upper, (b + 1u) << BIN_SHIFT);   // count(>= hi) == 0
+      if (count_from(lo, upper) <= CHUNK) hi = lo;
+      while (hi - lo > 1u) {
+        const unsigned mid = lo + ((hi - lo) >> 1);
+        if (count_from(mid, upper) <= CHUNK) hi = mid; else lo = mid;
+      }
+      cut = hi;
+    } else {
+      cut = max((unsigned)(bU - r_cut) << BIN_SHIFT, lowb);
+    }
+    if (cut >= upper) {                           // more than CHUNK candidates share one value: cannot be ordered in a chunk
+      if (tid == 0) { atomicExch(a.overflow, 1); s_done = 1; }
+      __syncthreads();
+      break;
+    }
     // --- gather chunk
+    const unsigned long long cutk = (unsigned long long)cut << 32, upk = (unsigned long long)upper << 32;
     if (tid == 0) s_cnt = 0;
     for (int i = tid; i < CHUNK; i += 1024) keys[i] = 0ull;
     __syncthreads();
     for (int i = tid; i < n; i += 1024) {
       const unsigned long long k = c[i];
-      if (k >= cut && k < upper) { const int p = atomicAdd(&s_cnt, 1); if (p < CHUNK) keys[p] = k; }
+      if (k >= cutk && k < upk) { const int p = atomicAdd(&s_cnt, 1); if (p < CHUNK) keys[p] = k; }
     }
     __syncthreads();
     const int m = min(s_cnt, CHUNK);
-    // --- bitonic sort, descending
-    for (int k2 = 2; k2 <= CHUNK; k2 <<= 1) {
+    // --- bitonic sort, descending, of the smallest power of two >= m (the keys after m are 0)
+    int P = 2;
+    while (P < m) P <<= 1;
+    for (int k2 = 2; k2 <= P; k2 <<= 1) {
       for (int j = k2 >> 1; j > 0; j >>= 1) {
-        for (int i = tid; i < CHUNK; i += 1024) {
+        for (int i = tid; i < P; i += 1024) {
           const int ixj = i ^ j;
           if (ixj > i) {
             const unsigned long long A = keys[i], B = keys[ixj];
@@ -294,9 +347,9 @@ __global__ void __launch_bounds__(1024) select_kernel(SelArgs a) {
       }
       if (tid == 0) {
         s_acc = acc;
-        const bool exhausted = (cut <= lowk);
-        s_done = (acc >= want) || exhausted || m == 0;
+        s_done = (acc >= want) || cut <= lowb;    // a chunk may be empty (the end bins over-count): only the threshold ends
         s_upper = cut;
+        s_rover = INT_MAX; s_rtgt = INT_MAX;
       }
     }
     __syncthreads();
@@ -335,9 +388,11 @@ __global__ void fill_kernel(uint8_t* p, size_t per_seq, const int* enable, uint8
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < per_seq / 16; i += (size_t)gridDim.x * blockDim.x) q[i] = vv;
 }
 
-__global__ void reset_detect_kernel(int* eig_max_key, int* n_cand, int n) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) { eig_max_key[i] = INT_MIN; n_cand[i] = 0; }
+// grid (LVB_CAND_BINS / 256, n)
+__global__ void reset_detect_kernel(int* eig_max_key, int* n_cand, int* hist) {
+  const int s = blockIdx.y;
+  hist[(size_t)s * LVB_CAND_BINS + blockIdx.x * 256 + threadIdx.x] = 0;
+  if (blockIdx.x == 0 && threadIdx.x == 0) { eig_max_key[s] = INT_MIN; n_cand[s] = 0; }
 }
 
 }  // namespace
@@ -352,7 +407,7 @@ int fe_detect_launch(LvbHandle* h, const uint8_t* pyr, int n_seq, const int* ena
   const int W = fe.W, H = fe.H;
   const uint8_t* mask = nullptr;
   LVB_PROF(h, "reset_detect_kernel");
-  reset_detect_kernel<<<(n_seq + 127) / 128, 128, 0, st>>>(fe.eig_max, fe.n_cand, n_seq);
+  reset_detect_kernel<<<dim3(LVB_CAND_BINS / 256, n_seq), 256, 0, st>>>(fe.eig_max, fe.n_cand, fe.cand_hist);
   LVB_LAUNCH_CHECK(h);
   if (ext_mask) mask = ext_mask;
   else if (use_mask) {
@@ -365,11 +420,11 @@ int fe_detect_launch(LvbHandle* h, const uint8_t* pyr, int n_seq, const int* ena
     mask = fe.mask;
   }
   CornerArgs ca; ca.pyr = pyr; ca.L = fe.L; ca.mask = mask; ca.eig = eig_out; ca.eig_max_key = fe.eig_max; ca.cand = fe.cand; ca.n_cand = fe.n_cand;
-  ca.cap = fe.cand_cap; ca.enable = enable;
+  ca.cap = fe.cand_cap; ca.hist = fe.cand_hist; ca.enable = enable;
   LVB_PROF(h, "corner_kernel");
   corner_kernel<<<dim3((W + TW - 1) / TW, (H + TH - 1) / TH, n_seq), 256, 0, st>>>(ca);
   LVB_LAUNCH_CHECK(h);
-  SelArgs sa; sa.cand = fe.cand; sa.n_cand = fe.n_cand; sa.cap = fe.cand_cap; sa.want = want; sa.W = W;
+  SelArgs sa; sa.cand = fe.cand; sa.n_cand = fe.n_cand; sa.cap = fe.cand_cap; sa.hist = fe.cand_hist; sa.want = want; sa.W = W;
   sa.min_dist = h->cfg.min_distance; sa.stride = fe.N; sa.out = out; sa.out_n = out_n; sa.overflow = fe.overflow; sa.enable = enable; sa.eig_max_key = fe.eig_max;
   LVB_PROF(h, "select_kernel");
   select_kernel<<<n_seq, 1024, 0, st>>>(sa);

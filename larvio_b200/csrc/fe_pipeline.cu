@@ -51,7 +51,7 @@ int fe_alloc(LvbHandle* h) {
   DA(fe.want, S); DA(fe.mask_n, S);
   DA(fe.mask, S * npx); DA(fe.eig_max, S);
   fe.cand_cap = 65536;                 // local maxima above 1 % of their tile's maximum (a superset of the final candidates)
-  DA(fe.cand, S * (size_t)fe.cand_cap); DA(fe.n_cand, S); DA(fe.overflow, 1); DA(fe.stats, 16);
+  DA(fe.cand, S * (size_t)fe.cand_cap); DA(fe.n_cand, S); DA(fe.cand_hist, S * LVB_CAND_BINS); DA(fe.overflow, 1); DA(fe.stats, 16);
   DA(fe.det_pts, S * N); DA(fe.det_n, S);
   DA(fe.msg, S * N); DA(fe.msg_n, S); DA(fe.has_msg, S); DA(fe.msg_t, S);
   fe.cur = 0;

@@ -175,6 +175,32 @@ extern "C" int lvbk_pyramid(LvbHandle* h, const uint8_t* images, int n, uint8_t*
   return LVB_OK;
 }
 
+// Level `level` of the pyramid lvbk_pyramid builds, WITH its LVB_PAD-wide REFLECT_101 pad: out [n][h + 2 LVB_PAD][w + 2 LVB_PAD].
+extern "C" int lvbk_pyramid_padded(LvbHandle* h, const uint8_t* images, int n, int level, uint8_t* out) {
+  if (!h || !images || !out || n <= 0) return lvb_set_err(LVB_E_ARG, "lvbk_pyramid_padded: bad argument");
+  LvbFrontEnd& fe = h->fe;
+  if (level < 0 || level >= fe.L.n_levels) return lvb_set_err(LVB_E_ARG, "lvbk_pyramid_padded: level %d outside [0, %d)", level, fe.L.n_levels);
+  LVB_CUDA(cudaSetDevice(h->device));
+  TmpBuf tb;
+  const size_t npx = (size_t)fe.W * fe.H;
+  uint8_t* d_img = tb.get<uint8_t>(npx * n);
+  uint8_t* d_pyr = tb.get<uint8_t>(fe.L.bytes_per_seq * n);
+  uint8_t* d_lut = tb.get<uint8_t>((size_t)n * 64 * 256);
+  if (!d_img || !d_pyr || !d_lut) return lvb_set_err(LVB_E_CUDA, "lvbk_pyramid_padded: cudaMalloc failed");
+  LVB_CUDA(cudaMemcpyAsync(d_img, images, npx * n, cudaMemcpyHostToDevice, h->stream));
+  uint8_t* saved = fe.lut; fe.lut = d_lut;
+  int rc = fe_build_pyramid(h, d_img, n, d_pyr, nullptr);
+  fe.lut = saved;
+  if (rc != LVB_OK) return rc;
+  const LvbLevel& lv = fe.L.lv[level];
+  const size_t row = (size_t)lv.w + 2 * LVB_PAD, rows = (size_t)lv.h + 2 * LVB_PAD;
+  for (int s = 0; s < n; ++s)
+    LVB_CUDA(cudaMemcpy2DAsync(out + (size_t)s * rows * row, row, d_pyr + (size_t)s * fe.L.bytes_per_seq + lv.offset, lv.pitch,
+                               row, rows, cudaMemcpyDeviceToHost, h->stream));
+  LVB_CUDA(cudaStreamSynchronize(h->stream));
+  return LVB_OK;
+}
+
 extern "C" int lvbk_lk(LvbHandle* h, const uint8_t* prev, const uint8_t* next, int n, int m,
                        const float* prev_pts, float* next_pts, uint8_t* status) {
   if (!h || !prev || !next || n <= 0 || m <= 0) return lvb_set_err(LVB_E_ARG, "lvbk_lk: bad argument");

@@ -9,6 +9,7 @@
 #include <vector>
 #include "../../include/larvio_b200.h"
 
+#define LVB_CAND_BINS 4096  // corner candidate histogram bins: value bits >> 19 (8 exponent + 4 mantissa bits)
 #define LVB_PAD 24          // pyramid level padding (>= patch_size 21 + 1, see App. C-10)
 #define LVB_MAX_LEVELS 4
 #define LVB_DESC_BYTES 32
@@ -27,6 +28,12 @@ struct LvbPyramidLayout {
 };
 
 // pointer to pixel (0,0) of level l of sequence s in pyramid block `base`
+// REFLECT_101 index of p in [0, n) (for -n < p < 2n - 1): the border rule of every front-end filter
+__host__ __device__ inline int lvb_reflect101(int p, int n) {
+  if (p < 0) p = -p;
+  if (p >= n) p = 2 * n - 2 - p;
+  return p;
+}
 __host__ __device__ inline const uint8_t* lvb_level_origin(const uint8_t* base, const LvbPyramidLayout& L,
                                                            int s, int l) {
   return base + (size_t)s * L.bytes_per_seq + L.lv[l].offset + (size_t)LVB_PAD * L.lv[l].pitch + LVB_PAD;
@@ -86,6 +93,7 @@ struct LvbFrontEnd {
   int* eig_max;                   // [S] ordered-int key of the masked max
   unsigned long long* cand;       // [S][cand_cap] packed (value bits<<32 | pixel index)
   int* n_cand; int cand_cap;
+  int* cand_hist;                 // [S][LVB_CAND_BINS] candidate count per value-bits bin (bits 30..19 of the positive float)
   int* overflow;                  // [1] sticky capacity-overflow flag
   unsigned long long* stats;      // [16] work counters: 0 LK point-tracks, 1 ORB descriptors, 2 detector runs, 3 published msgs,
                                   //      4 EKF updates, 5 sum r, 6 sum r*d*d, 7 sum stacked rows, 8 QR runs, 9 sum R*c*c

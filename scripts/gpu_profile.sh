@@ -9,7 +9,7 @@ python scripts/profile_driver.py gen
 ncu --profile-from-start off --metrics gpu__time_duration.sum --clock-control none --csv --log-file gpurun_out/launches_${TAG}.csv \
     python scripts/profile_driver.py run > gpurun_out/ncu_launches_${TAG}.log 2>&1
 tail -2 gpurun_out/ncu_launches_${TAG}.log
-for K in ${KERNELS:-lk_kernel ransac_kernel be_qr_kernel be_gemm_kernel orb_gate_kernel be_propagate_kernel be_stack_kernel be_feature_kernel select_kernel corner_kernel be_colscan_kernel be_add_obs_kernel be_chol_kernel be_trsm_kernel clahe_apply_kernel blur7_kernel pyrdown_kernel}; do
+for K in ${KERNELS:-lk_kernel ransac_kernel be_qr_kernel be_gemm_kernel orb_gate_kernel be_propagate_kernel be_stack_kernel be_feature_kernel select_kernel corner_kernel be_colscan_kernel be_add_obs_kernel be_chol_kernel be_trsm_kernel clahe_pyr_blur_kernel pyrdown_kernel}; do
   ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:^$K -c ${NCAP:-6} -o gpurun_out/prof_${K}_${TAG} -f \
       python scripts/profile_driver.py run > gpurun_out/ncu_${K}_${TAG}.log 2>&1
   tail -1 gpurun_out/ncu_${K}_${TAG}.log
